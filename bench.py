@@ -171,6 +171,49 @@ def reference_note_path(workload, gpus):
     return "/tmp/gv_b200_reference_%s_n%d.json" % (workload, gpus)
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(directory, arrays):
+    """Writes `arrays` (name -> 2-D array of vertex / entity / relation ids) as DIR/<name>.npy in float64, which holds
+    every id exactly.  Arrays that together exceed DUMP_BYTES are cut down to a fixed, seeded sample of rows (sorted,
+    drawn from the row count alone), so that two builds of the project run with the same arguments can be compared
+    output for output."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(8 * a.size for a in arrays.values())
+    budget = DUMP_BYTES - 4096 * len(arrays)  # room for the .npy headers
+    for name, matrix in arrays.items():
+        rows = matrix.shape[0]
+        keep = rows if total <= budget else max(1, int(rows * budget // total))
+        if keep < rows:
+            matrix = matrix[np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(matrix, dtype=np.float64))
+
+
+def sample_pools(pool_function, handle, num_partition, pool_id, width):
+    """The two sample pools after the timed steps, every (head, tail) block in order: the one the last step trained on
+    and the one the samplers filled during it.  Training itself is Hogwild -- concurrent updates of a row race, as in
+    the reference -- so the embeddings differ from run to run by the updates lost to races; the pools are what the
+    timed path computes deterministically from its inputs."""
+    from graphvite_b200 import _lib
+    out = {}
+    for name, pool in (("trained_pool", pool_id), ("next_pool", pool_id ^ 1)):
+        blocks = []
+        for head in range(num_partition):
+            for tail in range(num_partition):
+                count = pool_function(handle, pool, head, tail, None)  # 0: a tail partition another rank holds
+                if count < 0:
+                    raise _lib.GVError(_lib.last_error())
+                if count == 0:
+                    continue
+                block = np.zeros((count, width), dtype=np.uint32)
+                if pool_function(handle, pool, head, tail, block.ctypes.data) < 0:
+                    raise _lib.GVError(_lib.last_error())
+                blocks.append(block)
+        out[name] = np.concatenate(blocks)
+    return out
+
+
 # --------------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------------
@@ -321,6 +364,9 @@ def run_ours(args, cfg):
     after = solver.stats
     seconds = max_over_ranks(seconds)
     _lib.check(lib.gv_solver_train_end(handle))
+    if args.dump_outputs and rank == 0:  # pairs {tail, head}
+        dump_outputs(args.dump_outputs, sample_pools(lib.gv_solver_pool, handle, solver.num_partition,
+                                                     solver.pool_id, 2))
     value = args.steps * edges_per_step * world / seconds
 
     # roofline of the dominant kernel (the train kernel): algorithmic bytes / CUDA-event time of its launches
@@ -531,6 +577,9 @@ def run_ours_kg(args, cfg):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         seconds, kernel_seconds = float(t[0].item()), float(t[1].item())
     _lib.check(lib.gv_kg_solver_train_end(handle))
+    if args.dump_outputs and rank == 0:  # triplets {relation, tail, head}
+        dump_outputs(args.dump_outputs, sample_pools(lib.gv_kg_solver_pool, handle, solver.num_partition,
+                                                     solver.pool_id, 3))
     per_positive = kg_bytes_per_positive(cfg["dim"], cfg["num_negative"], 2)
     peak, peak_kind = measured_peak()
     achieved = positives * per_positive / max(kernel_seconds, 1e-12) / 1e9
@@ -708,6 +757,9 @@ def main():
     parser.add_argument("--parity-timeout", type=int, default=300, help="deadline of the parity self-check in seconds")
     parser.add_argument("--partitions", type=int, default=0, help="num_partition (0 = auto; diagnosis only)")
     parser.add_argument("--watchdog", type=int, default=1500, help="abort after this many seconds (0 = never)")
+    parser.add_argument("--dump-outputs", default="", metavar="DIR",
+                        help="write the sample pools of the last timed step as DIR/<name>.npy (float64 ids, at most "
+                             "64 MB in all: a fixed, seeded sample of rows where the pools are larger)")
     args = parser.parse_args()
     if args.watchdog > 0:
         start_watchdog(args.watchdog)

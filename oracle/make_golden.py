@@ -233,6 +233,23 @@ def write_solver_cases(lib, out_dir, toy, only):
     print("golden vectors written to", out_dir)
 
 
+# Solver runs whose embeddings tests/test_emulated_reference.py compares with the oracle's.  Only the emulated
+# reference processes a batch in order, like the oracle, so these are recorded with --emulated:
+#     python oracle/make_golden.py --emulated --oracle-check tests/golden
+# Both embedding matrices are kept whole, and predict on the run's pairs.
+ORACLE_CHECK_CASES = ("line_p1", "edge_p2", "node2vec_p1")
+
+
+def write_oracle_check_cases(lib, out_dir, toy):
+    import tempfile
+    with tempfile.TemporaryDirectory() as tmp:
+        write_solver_cases(lib, tmp, toy, set(ORACLE_CHECK_CASES))
+        for name in ORACLE_CHECK_CASES:
+            g = np.load(os.path.join(tmp, "solver_%s.npz" % name))
+            np.savez_compressed(os.path.join(out_dir, "emu_reference_solver_%s.npz" % name), vertex=g["vertex"],
+                                context=g["context"], logits=g["logits"])
+
+
 def write_kernel_cases(lib, out_dir):
     # ---- the reference kernels on race-free batches ---------------------------------------------
     for dim in (32, 128):
@@ -262,5 +279,8 @@ def write_kernel_cases(lib, out_dir):
 
 
 if __name__ == "__main__":
-    arguments = [a for a in sys.argv[1:] if a != "--emulated"]
+    arguments = [a for a in sys.argv[1:] if a not in ("--emulated", "--oracle-check")]
+    if "--oracle-check" in sys.argv:
+        write_oracle_check_cases(load_harness(), arguments[0], os.path.join(GOLDEN, "toy_graph.txt"))
+        sys.exit(0)
     main(arguments[0] if arguments else os.path.join(ROOT, "gpurun_out", "golden"), set(arguments[1:]) or None)

@@ -46,4 +46,6 @@ bench.ClockSampler = NoClocks
 bench.make_solver = make_solver
 sys.argv = ["bench.py", "--workload", "toy", "--gpus", os.environ.get("WORLD_SIZE", "1"), "--steps", "4", "--warmup",
             "2", "--no-cpu-baseline", "--watchdog", "0"]
+if os.environ.get("GV_BENCH_DUMP"):
+    sys.argv += ["--dump-outputs", os.environ["GV_BENCH_DUMP"]]
 bench.main()

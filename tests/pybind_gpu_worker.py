@@ -21,31 +21,39 @@ def load():
     return m
 
 
-def graph_solver_matches_the_ctypes_mirror(module):
+def graph_solver_matches_the_ctypes_mirror(module, repeat=4):
+    """Hogwild training on the toy graph loses a varying share of racing updates, and which share follows the state
+    of the GPU (single runs spread by several percent, drifting over a process's first runs), so the two front ends
+    train alternately and their embedding norms are compared as means over `repeat` runs of each."""
     import graphvite_b200 as gv
     from graphvite_b200 import _lib
     train = dict(model="LINE", num_epoch=40, augmentation_step=2, random_walk_length=5, random_walk_batch_size=10)
 
-    _lib.lib.gv_reset_global_engine(5489)
-    graph = module.graph.Graph_j()
-    graph.load(TOY)
-    solver = module.solver.GraphSolver_32_f_j([0], 1, 0)
-    solver.build(graph, module.optimizer.SGD(0.025, 0.005), 1, 1, 500, 4)
-    assert (solver.num_partition, solver.batch_size, solver.episode_size, solver.num_negative) == (1, 500, 4, 1)
-    solver.train(**train)
-    assert solver.model == "LINE" and solver.augmentation_step == 2
-    vertex, context = solver.vertex_embeddings, solver.context_embeddings
-    assert vertex.shape == (graph.num_vertex, 32) and vertex.dtype == np.float32 and not vertex.flags.owndata
+    norms, mirror_norms = [], []
+    for _ in range(repeat):
+        _lib.lib.gv_reset_global_engine(5489)
+        graph = module.graph.Graph_j()
+        graph.load(TOY)
+        solver = module.solver.GraphSolver_32_f_j([0], 1, 0)
+        solver.build(graph, module.optimizer.SGD(0.025, 0.005), 1, 1, 500, 4)
+        assert (solver.num_partition, solver.batch_size, solver.episode_size, solver.num_negative) == (1, 500, 4, 1)
+        solver.train(**train)
+        assert solver.model == "LINE" and solver.augmentation_step == 2
+        vertex, context = solver.vertex_embeddings, solver.context_embeddings
+        assert vertex.shape == (graph.num_vertex, 32) and vertex.dtype == np.float32 and not vertex.flags.owndata
+        norms.append((float(np.linalg.norm(vertex)), float(np.linalg.norm(context))))
 
-    _lib.lib.gv_reset_global_engine(5489)
-    graph2 = gv.graph.Graph()
-    graph2.load(TOY)
-    mirror = gv.solver.GraphSolver(32, device_ids=[0], num_sampler_per_worker=1)
-    mirror.build(graph2, gv.optimizer.SGD(0.025, 0.005), 1, 1, 500, 4)
-    mirror.train(**train)
-    for ours, theirs in ((vertex, mirror.vertex_embeddings), (context, mirror.context_embeddings)):
-        a, b = float(np.linalg.norm(ours)), float(np.linalg.norm(theirs))
-        assert np.isfinite(a) and abs(a - b) <= 0.05 * b, (a, b)
+        _lib.lib.gv_reset_global_engine(5489)
+        graph2 = gv.graph.Graph()
+        graph2.load(TOY)
+        mirror = gv.solver.GraphSolver(32, device_ids=[0], num_sampler_per_worker=1)
+        mirror.build(graph2, gv.optimizer.SGD(0.025, 0.005), 1, 1, 500, 4)
+        mirror.train(**train)
+        mirror_norms.append((float(np.linalg.norm(mirror.vertex_embeddings)),
+                             float(np.linalg.norm(mirror.context_embeddings))))
+        mirror.close()
+    for a, b in zip(np.mean(norms, axis=0), np.mean(mirror_norms, axis=0)):
+        assert np.isfinite(a) and abs(a - b) <= 0.05 * b, (norms, mirror_norms)
     # the views alias the solver's memory: predict sees an edit made through them
     pairs = np.array([[0, 1], [2, 3]], dtype=np.uint32)
     before = solver.predict(pairs)

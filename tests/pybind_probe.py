@@ -1,6 +1,7 @@
 """Loads ONE pybind11 module named `libgraphvite` from the path in argv[1] and prints what tests/test_pybind_module.py
 compares, as JSON.  A separate process per module: two extension modules with the same name (the reference's and
 ours) cannot live in one interpreter -- their `libgraphvite.solver` submodules would share one sys.modules entry."""
+import hashlib
 import importlib.util
 import json
 import os
@@ -9,6 +10,11 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TOY = os.path.join(ROOT, "tests", "golden", "toy_graph.txt")
+
+
+def file_digest(path):
+    with open(path, "rb") as fin:
+        return hashlib.sha256(fin.read()).hexdigest()
 
 
 def public(obj):
@@ -35,7 +41,7 @@ def main():
         g.save(os.path.join(tmp, "toy.txt"), True, False)
         graphs["file"] = {"num_vertex": g.num_vertex, "num_edge": g.num_edge, "as_undirected": g.as_undirected,
                           "normalization": g.normalization, "id2name": list(g.id2name), "name2id": dict(g.name2id),
-                          "saved": open(os.path.join(tmp, "toy.txt")).read()}
+                          "saved_sha256": file_digest(os.path.join(tmp, "toy.txt"))}
         g.load([("a", "b"), ("b", "c"), ("c", "a"), ("a", "a")], as_undirected=False)
         graphs["edge_list"] = {"num_vertex": g.num_vertex, "num_edge": g.num_edge, "name2id": dict(g.name2id)}
         g.load([("x", "y", 2.0), ("y", "z", 0.5)], normalization=True)

@@ -4,7 +4,13 @@ recorded from the same reference on a real B200 (tests/golden/, oracle/make_gold
 cuRAND streams, alias tables, partitions, BOTH sample pools and the last negatives of full solver runs -- must be
 bit-identical to what the hardware produced, and the train kernels (race-free batches) equal up to the rounding of
 libm / FMA contraction.  (Embeddings of the solver runs are not compared: the B200 run is Hogwild, the emulation
-processes a batch in order.)  Skipped where the emulated reference is not built (it needs /root/reference)."""
+processes a batch in order.)  Skipped where the emulated reference is not built (`make -C oracle ref_emu` needs the
+reference's sources).
+
+The emulation processes a batch in order, like the oracle, so its solver runs also pin the oracle's training arithmetic
+float for float.  That comparison does not need the reference at hand: what the emulated reference trained (both
+embedding matrices, and predict) is stored in tests/golden/emu_reference_*.npz
+(`python oracle/make_golden.py --emulated --oracle-check tests/golden`)."""
 import os
 import subprocess
 import sys
@@ -21,7 +27,10 @@ SOLVER_CASES = ["line_p1", "edge_p2", "node2vec_p1"]
 if os.environ.get("GV_EMU_FULL") == "1":
     SOLVER_CASES += ["line_p2_s3", "deepwalk_p1", "line_p3_adam", "node2vec_p2"]
 
-pytestmark = pytest.mark.skipif(not os.path.exists(LIBRARY), reason="oracle/_ref/libref_harness_emu.so is not built")
+needs_emulated_reference = pytest.mark.skipif(not os.path.exists(LIBRARY),
+                                              reason="oracle/_ref/libref_harness_emu.so is not built")
+# solver runs of the emulated reference stored for the oracle comparison (oracle/make_golden.py ORACLE_CHECK_CASES)
+RECORDED_CASES = ["line_p1", "edge_p2", "node2vec_p1"]
 
 
 @pytest.fixture(scope="module")
@@ -56,32 +65,46 @@ def compare(regenerated, name, float_tolerance=None, skip=()):
             np.testing.assert_allclose(a, b, err_msg="%s:%s" % (name, key), **float_tolerance)
 
 
+@needs_emulated_reference
 @pytest.mark.parametrize("name", ["curand.npz", "alias.npz", "graph_u0_n0.npz", "graph_u0_n1.npz", "graph_u1_n0.npz",
                                   "graph_u1_n1.npz"])
 def test_host_side_fixtures_regenerate_identically(regenerated, name):
     compare(regenerated, name)
 
 
+@needs_emulated_reference
 @pytest.mark.parametrize("optimizer", ["SGD", "Momentum", "AdaGrad", "RMSprop", "Adam"])
 @pytest.mark.parametrize("dim", [32, 128])
 def test_train_kernels_match_the_b200_to_rounding(regenerated, dim, optimizer):
     compare(regenerated, "kernel_d%d_%s.npz" % (dim, optimizer), float_tolerance=dict(rtol=2e-5, atol=2e-6))
 
 
+@needs_emulated_reference
 @pytest.mark.parametrize("case", SOLVER_CASES)
 def test_solver_runs_reproduce_the_b200s_integer_state(regenerated, case):
     # vertex / context / loss / logits: Hogwild on the B200, in order here; edge_prob is float but host-built
     compare(regenerated, "solver_%s.npz" % case, skip=("vertex", "context", "loss", "logits"))
 
 
-@pytest.mark.parametrize("case", SOLVER_CASES)
-def test_oracle_training_arithmetic_equals_the_references_in_order(regenerated, case):
+@needs_emulated_reference
+@pytest.mark.parametrize("case", RECORDED_CASES)
+def test_stored_solver_runs_are_the_emulated_references(regenerated, case):
+    """provenance of tests/golden/emu_reference_solver_*.npz: the emulated reference regenerates them bit for bit"""
+    ours, stored = np.load(os.path.join(regenerated, "solver_%s.npz" % case)), \
+        np.load(os.path.join(GOLDEN, "emu_reference_solver_%s.npz" % case))
+    for key in ("vertex", "context", "logits"):
+        np.testing.assert_array_equal(ours[key], stored[key], err_msg=key)
+
+
+@pytest.mark.parametrize("case", RECORDED_CASES)
+def test_oracle_training_arithmetic_equals_the_references_in_order(case):
     """On the B200 the reference's solver runs are Hogwild, so tests/test_oracle_golden.py can pin the oracle's
     integer state only.  The emulation processes a batch in order (one warp per sample, warps one after another) --
     the oracle's order -- so here the oracle's whole training run is compared with the reference's float for float:
     vertex / context embeddings, the last batch's losses and predict."""
     import oracle_lib as O
-    g = np.load(os.path.join(regenerated, "solver_%s.npz" % case))
+    g = np.load(os.path.join(GOLDEN, "solver_%s.npz" % case))  # configuration and predict pairs of the run
+    recorded = np.load(os.path.join(GOLDEN, "emu_reference_solver_%s.npz" % case))
     cfg = {key[4:]: g[key].item() for key in g.files if key.startswith("cfg_")}
     graph = O.OracleGraph(os.path.join(GOLDEN, "toy_graph.txt"))
     solver = O.OracleSolver(graph, cfg["dim"], 1, cfg["S"])
@@ -90,6 +113,6 @@ def test_oracle_training_arithmetic_equals_the_references_in_order(regenerated, 
                  random_walk_length=cfg["L"], random_walk_batch_size=cfg["wb"], p=cfg.get("p", 1.0),
                  q=cfg.get("q", 1.0))
     tolerance = dict(rtol=1e-4, atol=1e-7)
-    np.testing.assert_allclose(solver.embeddings(0), g["vertex"], **tolerance)
-    np.testing.assert_allclose(solver.embeddings(1), g["context"], **tolerance)
-    np.testing.assert_allclose(solver.predict(g["pairs"]), g["logits"], rtol=1e-4, atol=1e-6)
+    np.testing.assert_allclose(solver.embeddings(0), recorded["vertex"], **tolerance)
+    np.testing.assert_allclose(solver.embeddings(1), recorded["context"], **tolerance)
+    np.testing.assert_allclose(solver.predict(g["pairs"]), recorded["logits"], rtol=1e-4, atol=1e-6)

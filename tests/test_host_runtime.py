@@ -222,20 +222,19 @@ def test_yaml_config_loading(tmp_path):
     """the reference's quick-start configuration loads unchanged except for the dataset placeholders"""
     import yaml
     from graphvite_b200 import cmd, optimizer, auto
-    reference = "/root/reference/config/demo/quick_start.yaml"
-    if os.path.exists(reference):
-        cfg = yaml.safe_load(open(reference))
-    else:  # the same content (config/demo/quick_start.yaml), for boxes without /root/reference
-        cfg = {"application": "graph", "resource": {"gpus": [0], "cpu_per_gpu": 8, "dim": 128},
-               "format": {"delimiters": " \t\r\n", "comment": "#"},
-               "graph": {"file_name": "<blogcatalog.train>", "as_undirected": True},
-               "build": {"optimizer": {"type": "SGD", "lr": 0.025, "weight_decay": 0.005}, "num_partition": "auto",
-                         "num_negative": 1, "batch_size": 100000, "episode_size": 500},
-               "train": {"model": "LINE", "num_epoch": 2000, "negative_weight": 5, "augmentation_step": 2,
-                         "random_walk_length": 40, "random_walk_batch_size": 100, "log_frequency": 1000},
-               "evaluate": [{"task": "link prediction", "file_name": "<blogcatalog.test>",
-                             "filter_file": "<blogcatalog.train>"}],
-               "save": {"file_name": "line_blogcatalog.pkl"}}
+    # the content of the reference's config/demo/quick_start.yaml
+    cfg = {"application": "graph", "resource": {"gpus": [0], "cpu_per_gpu": 8, "dim": 128},
+           "format": {"delimiters": " \t\r\n", "comment": "#"},
+           "graph": {"file_name": "<blogcatalog.train>", "as_undirected": True},
+           "build": {"optimizer": {"type": "SGD", "lr": 0.025, "weight_decay": 0.005}, "num_partition": "auto",
+                     "num_negative": 1, "batch_size": 100000, "episode_size": 500},
+           "train": {"model": "LINE", "num_epoch": 2000, "negative_weight": 5, "augmentation_step": 2,
+                     "random_walk_length": 40, "random_walk_batch_size": 100, "log_frequency": 1000},
+           "evaluate": [{"task": "link prediction", "file_name": "<blogcatalog.test>",
+                         "filter_file": "<blogcatalog.train>"},
+                        {"task": "node classification", "file_name": "<blogcatalog.label>", "portions": [0.2],
+                         "times": 1}],
+           "save": {"file_name": "line_blogcatalog.pkl"}}
     path = tmp_path / "quick_start.yaml"
     path.write_text(yaml.safe_dump(cfg))
     with pytest.raises(ValueError, match="dataset placeholder"):

@@ -1,13 +1,14 @@
 """CPU checks of the knowledge-graph oracle (oracle/gv_oracle_kg.cpp).
 
-The loader is pinned against the live reference object (where oracle/_ref exists) and against the
-product's loader.  The solver and kernels are NOT yet pinned against reference output (their goldens
-need a GPU, oracle/make_golden.py kg_*): what is checked here is internal consistency -- backward is
-the gradient of forward, the tied schedule covers every block exactly once without sharing a partition
-inside a step, pools hold valid triplets of the right block, training lowers the loss and ranks true
+The loader is pinned against what the reference object loaded (tests/golden/reference_surface.json, recorded by
+oracle/record_reference_surface.py) and against the product's loader.  The solver and kernels are NOT yet pinned
+against reference output (their goldens need a GPU, oracle/make_golden.py kg_*): what is checked here is internal
+consistency -- backward is the gradient of forward, the tied schedule covers every block exactly once without sharing
+a partition inside a step, pools hold valid triplets of the right block, training lowers the loss and ranks true
 triplets first -- so that a wrong restatement is caught before it is used to judge CUDA code.
 """
-import importlib.util
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -17,7 +18,7 @@ import oracle_kg_lib as K
 import oracle_lib as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_PATH = os.path.join(ROOT, "oracle", "_ref", "libgraphvite.so")
+RECORDED = os.path.join(ROOT, "tests", "golden", "reference_surface.json")
 
 
 def toy_triplets(seed=0, num_entity=60, num_relation=5, num_triplet=900):
@@ -55,25 +56,32 @@ def test_loader_matches_the_product_loader(tmp_path, normalization):
             np.testing.assert_array_equal(ours, theirs)  # floats too: same accumulation order
 
 
-@pytest.mark.skipif(not os.path.exists(REF_PATH), reason="oracle/_ref/libgraphvite.so is not built")
-def test_loader_matches_the_live_reference(tmp_path):
-    spec = importlib.util.spec_from_file_location("libgraphvite", REF_PATH)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    ref.init_logging(ref.ERROR, "", False)
-    triplets = toy_triplets(3)
-    theirs = ref.graph.KnowledgeGraph_j()
-    theirs.load(triplets, False)
-    oracle = K.OracleKnowledgeGraph(triplets)
-    assert (theirs.num_vertex, theirs.num_edge, theirs.num_relation) == \
-        (oracle.num_vertex, oracle.num_edge, oracle.num_relation)
-    assert list(theirs.id2entity) == oracle.id2entity() and list(theirs.id2relation) == oracle.id2relation()
-    path = str(tmp_path / "ref.txt")
-    theirs.save(path, True)  # anonymous: head, tail, int(weight) in flatten order
+def observe_toy_knowledge_graph(kg_class, tmp_path):
+    """what the reference's KnowledgeGraph made of toy_triplets(3): counts, id maps, and digests of the head and
+    tail columns of its anonymous save (head, tail, int(weight) in flatten order)"""
+    graph = kg_class()
+    graph.load(toy_triplets(3), False)
+    path = str(tmp_path / "anonymous.txt")
+    graph.save(path, True)
     columns = np.loadtxt(path, dtype=np.int64, ndmin=2)
+    return {"counts": [graph.num_vertex, graph.num_edge, graph.num_relation], "id2entity": list(graph.id2entity),
+            "id2relation": list(graph.id2relation), "heads": int64_digest(columns[:, 0]),
+            "tails": int64_digest(columns[:, 1])}
+
+
+def int64_digest(values):
+    return hashlib.sha256(np.ascontiguousarray(values, dtype="<i8").tobytes()).hexdigest()
+
+
+def test_loader_matches_the_live_reference():
+    with open(RECORDED) as fin:
+        theirs = json.load(fin)["kg_toy_triplets"]
+    oracle = K.OracleKnowledgeGraph(toy_triplets(3))
+    assert theirs["counts"] == [oracle.num_vertex, oracle.num_edge, oracle.num_relation]
+    assert theirs["id2entity"] == oracle.id2entity() and theirs["id2relation"] == oracle.id2relation()
     h, t, r, w, _ = oracle.flat()
-    np.testing.assert_array_equal(columns[:, 0], h)
-    np.testing.assert_array_equal(columns[:, 1], t)
+    assert theirs["heads"] == int64_digest(h)
+    assert theirs["tails"] == int64_digest(t)
 
 
 # ---- models: backward is the gradient of forward ----------------------------------------------------

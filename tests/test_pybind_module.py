@@ -1,9 +1,10 @@
 """The compiled pybind11 module `libgraphvite` over the C ABI (graphvite_b200/csrc/pybind/libgraphvite.cpp ->
 graphvite_b200/pybind/libgraphvite.so): the surface a reference maintainer gets when `src/graphvite.cu`'s classes are
-swapped for libgv_b200.  Checked on CPU against the UNMODIFIED reference module (oracle/_ref/libgraphvite.so, when it
-was built here): same submodules and class names, the same argument names / order / defaults of every solver method
-(parsed from both modules' docstrings), the same optimizer objects, and a Graph that loads, maps and saves the same
-bytes.  Training through this module runs on the GPU box (tests/test_gpu_x_pybind.py)."""
+swapped for libgv_b200.  Checked on CPU against what tests/pybind_probe.py printed for the UNMODIFIED reference
+module (recorded in tests/golden/reference_pybind_probe.json): same submodules and class names, the same argument
+names / order / defaults of every solver method (parsed from both modules' docstrings), the same optimizer objects,
+and a Graph that loads, maps and saves the same bytes.  Training through this module runs on the GPU box
+(tests/test_gpu_x_pybind.py)."""
 import json
 import os
 import re
@@ -15,9 +16,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUR_PATH = os.path.join(ROOT, "graphvite_b200", "pybind", "libgraphvite.so")
-REF_PATH = os.path.join(ROOT, "oracle", "_ref", "libgraphvite.so")
+RECORDED = os.path.join(ROOT, "tests", "golden", "reference_pybind_probe.json")
 TOY = os.path.join(ROOT, "tests", "golden", "toy_graph.txt")
-needs_reference = pytest.mark.skipif(not os.path.exists(REF_PATH), reason="oracle/_ref/libgraphvite.so is not built")
 
 
 def probe(path):
@@ -45,7 +45,10 @@ def mine(ours):
 
 @pytest.fixture(scope="module")
 def theirs():
-    return probe(REF_PATH)
+    """tests/pybind_probe.py's output for the reference's module (python tests/pybind_probe.py
+    oracle/_ref/libgraphvite.so, built by `make -C oracle ref`)"""
+    with open(RECORDED) as fin:
+        return json.load(fin)
 
 
 def public(obj):
@@ -75,7 +78,6 @@ def test_module_layout(mine):
     assert mine["auto"] == 0 and mine["gib2"] == 2 << 30 and mine["dtype2name"]["uint32"] == "j"
 
 
-@needs_reference
 def test_same_names_as_the_reference_module(mine, theirs):
     skip = {"VisualizationSolver_2_f_j", "VisualizationSolver_3_f_j", "KNNGraph_j"}  # LargeVis: out of scope
     for sub in ("solver", "graph", "optimizer"):
@@ -110,7 +112,6 @@ def signature_of(doc, generated):
     return out[1:]  # drop self
 
 
-@needs_reference
 @pytest.mark.parametrize("method", ["GraphSolver_128_f_j.build", "GraphSolver_128_f_j.train",
                                     "GraphSolver_128_f_j.predict", "GraphSolver_128_f_j.clear",
                                     "KnowledgeGraphSolver_2048_f_j.build", "KnowledgeGraphSolver_2048_f_j.train",
@@ -123,19 +124,16 @@ def test_solver_method_signatures(mine, theirs, method):
         assert same_default(a, b), (method, name, a, b)
 
 
-@needs_reference
 @pytest.mark.parametrize("cls", ["GraphSolver_128_f_j", "KnowledgeGraphSolver_2048_f_j"])
 def test_solver_attributes_are_all_present(mine, theirs, cls):
     missing = set(theirs["attributes"][cls]) - set(mine["attributes"][cls])
     assert not missing, missing
 
 
-@needs_reference
 def test_graph_loads_maps_and_saves_like_the_reference(mine, theirs):
     assert mine["graphs"] == theirs["graphs"]  # counts, id2name, name2id, and the bytes save() writes
 
 
-@needs_reference
 def test_optimizer_objects(mine, theirs):
     assert set(mine["optimizers"]) == set(theirs["optimizers"])
     for name, reference in theirs["optimizers"].items():

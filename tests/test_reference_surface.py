@@ -1,14 +1,15 @@
-"""Drop-in surface checks against the UNMODIFIED reference module, when it was built in this
-container (oracle/_ref/libgraphvite.so, `make -C oracle ref`).  The pybind module imports without a
-GPU: its classes, docstring signatures, optimizer objects and the host-side Graph are all usable on
-CPU, so the mirror in graphvite_b200/ is compared with the real thing rather than with a reading of it.
+"""Drop-in surface checks against the UNMODIFIED reference module.  The pybind module imports without a GPU: its
+classes, docstring signatures, optimizer objects and the host-side Graph are all usable on CPU, so the mirror in
+graphvite_b200/ is compared with what the real thing did rather than with a reading of it.
 
-Skipped where the reference build is absent (the GPU box gets the prebuilt file with the snapshot;
-a clone without /root/reference has nothing to compare with).
+What the reference did is recorded in tests/golden/reference_surface.json by oracle/record_reference_surface.py (run
+where the reference module is built, `make -C oracle ref`): its public names and docstrings, its optimizer objects and
+learning-rate schedules, and for every loader scenario below the counts, the id maps and SHA-256 digests of the files
+its save() wrote.  The scenarios themselves (seeded inputs, `observe_*`) are defined here once and run on both.
 """
-import filecmp
-import importlib.util
+import hashlib
 import inspect
+import json
 import os
 import re
 
@@ -16,19 +17,14 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_PATH = os.path.join(ROOT, "oracle", "_ref", "libgraphvite.so")
+RECORDED = os.path.join(ROOT, "tests", "golden", "reference_surface.json")
 TOY = os.path.join(ROOT, "tests", "golden", "toy_graph.txt")
-
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_PATH), reason="oracle/_ref/libgraphvite.so is not built")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    spec = importlib.util.spec_from_file_location("libgraphvite", REF_PATH)
-    module = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(module)
-    module.init_logging(module.ERROR, "", False)
-    return module
+    with open(RECORDED) as fin:
+        return json.load(fin)
 
 
 @pytest.fixture(scope="module")
@@ -41,9 +37,9 @@ def public(obj):
     return {name for name in dir(obj) if not name.startswith("_")}
 
 
-def doc_signature(function):
+def doc_signature(doc):
     """[(name, default-or-None)] from the first docstring line pybind11 was given (bind.h)."""
-    head = function.__doc__.strip().split("\n")[0]
+    head = doc.strip().split("\n")[0]
     inside = re.match(r"\w+\((.*)\)$", head).group(1)
     out = []
     for item in filter(None, (s.strip() for s in inside.split(","))):
@@ -71,9 +67,26 @@ def same_default(ref_text, ours, gv):
     return float(ref_text) == float(ours)
 
 
+def digest(data):
+    return hashlib.sha256(data).hexdigest()
+
+
+def file_digest(path):
+    with open(path, "rb") as fin:
+        return digest(fin.read())
+
+
+def names_digest(names):
+    return digest("\n".join(names).encode())
+
+
+def int_digest(values):
+    return digest(np.ascontiguousarray(values, dtype="<i8").tobytes())
+
+
 @pytest.mark.parametrize("method", ["build", "train", "predict", "clear"])
 def test_solver_method_signatures(ref, gv, method):
-    theirs = doc_signature(getattr(ref.solver.GraphSolver_128_f_j, method))
+    theirs = doc_signature(ref["docs"]["GraphSolver_128_f_j." + method])
     ours = our_signature(getattr(gv.solver.GraphSolver, method))
     assert [n for n, _ in theirs] == [n for n, _ in ours]
     for (name, a), (_, b) in zip(theirs, ours):
@@ -83,20 +96,20 @@ def test_solver_method_signatures(ref, gv, method):
 def test_solver_attributes_are_all_present(ref, gv):
     from graphvite_b200 import solver as S
     ours = public(gv.solver.GraphSolver) | set(S._INT_ATTRIBUTES) | set(S._FLOAT_ATTRIBUTES)
-    missing = public(ref.solver.GraphSolver_128_f_j) - ours
+    missing = set(ref["public"]["GraphSolver_128_f_j"]) - ours
     assert not missing, missing
 
 
 def test_graph_surface(ref, gv):
-    assert public(ref.graph.Graph_j) <= public(gv.graph.Graph)
-    theirs = doc_signature(ref.graph.Graph_j.save)
+    assert set(ref["public"]["Graph_j"]) <= public(gv.graph.Graph)
+    theirs = doc_signature(ref["docs"]["Graph_j.save"])
     ours = our_signature(gv.graph.Graph.save)
     assert [n for n, _ in theirs] == [n for n, _ in ours]
     for (name, a), (_, b) in zip(theirs, ours):
         assert same_default(a, b, gv), (name, a, b)
-    assert gv.auto == ref.auto
+    assert gv.auto == ref["auto"]
     for unit in ("KiB", "MiB", "GiB"):
-        assert getattr(gv, unit)(3) == getattr(ref, unit)(3)
+        assert getattr(gv, unit)(3) == ref["units"][unit]
 
 
 OPTIMIZERS = {
@@ -106,32 +119,44 @@ OPTIMIZERS = {
     "RMSprop": ("lr", "weight_decay", "alpha", "epsilon"),
     "Adam": ("lr", "weight_decay", "beta1", "beta2", "epsilon"),
 }
+POSITIONAL = [0.5, 0.25, 0.75, 0.875, 0.125]
+
+
+def observe_optimizer(optimizer_module, name):
+    """what test_optimizer_defaults_and_positional_order compares, for either module's `optimizer`"""
+    fields = OPTIMIZERS[name]
+    default = getattr(optimizer_module, name)()
+    positional = getattr(optimizer_module, name)(*POSITIONAL[:len(fields)])
+    constant = getattr(optimizer_module, name)(schedule="constant")
+    return {"public": sorted(public(default)), "type": default.type,
+            "default": [float(np.float32(getattr(default, field))) for field in fields],
+            "positional": [float(getattr(positional, field)) for field in fields],
+            "schedule": default.schedule.type, "constant_schedule": constant.schedule.type}
 
 
 @pytest.mark.parametrize("name", sorted(OPTIMIZERS))
 def test_optimizer_defaults_and_positional_order(ref, gv, name):
-    fields = OPTIMIZERS[name]
-    theirs, ours = getattr(ref.optimizer, name)(), getattr(gv.optimizer, name)()
-    assert public(theirs) <= public(ours) | {"lr", "weight_decay", "schedule"}
-    assert theirs.type == ours.type
-    for field in fields:
-        assert np.float32(getattr(theirs, field)) == np.float32(getattr(ours, field)), field
-    assert theirs.schedule.type == ours.schedule.type == "linear"
+    theirs, ours = ref["optimizers"][name], observe_optimizer(gv.optimizer, name)
+    assert set(theirs["public"]) <= set(ours["public"]) | {"lr", "weight_decay", "schedule"}
+    assert theirs["type"] == ours["type"]
+    for field, a, b in zip(OPTIMIZERS[name], theirs["default"], ours["default"]):
+        assert a == b, field
+    assert theirs["schedule"] == ours["schedule"] == "linear"
     # positional construction assigns the same fields in the same order
-    values = [0.5, 0.25, 0.75, 0.875, 0.125][:len(fields)]
-    theirs, ours = getattr(ref.optimizer, name)(*values), getattr(gv.optimizer, name)(*values)
-    for field, value in zip(fields, values):
-        assert getattr(theirs, field) == getattr(ours, field) == value, field
-    theirs, ours = getattr(ref.optimizer, name)(schedule="constant"), getattr(gv.optimizer, name)(schedule="constant")
-    assert theirs.schedule.type == ours.schedule.type == "constant"
+    assert theirs["positional"] == ours["positional"] == POSITIONAL[:len(OPTIMIZERS[name])]
+    assert theirs["constant_schedule"] == ours["constant_schedule"] == "constant"
+
+
+LR_POINTS = ((0, 10), (3, 10), (9, 10), (10, 10), (1978, 1978), (12, 7))
+
+
+def observe_lr_schedules(optimizer_module):
+    return {kind: [float(np.float32(optimizer_module.LRSchedule(kind).schedule_function(batch_id, num_batch)))
+                   for batch_id, num_batch in LR_POINTS] for kind in ("constant", "linear")}
 
 
 def test_lr_schedules_agree(ref, gv):
-    for kind in ("constant", "linear"):
-        a, b = ref.optimizer.LRSchedule(kind), gv.optimizer.LRSchedule(kind)
-        for batch_id, num_batch in ((0, 10), (3, 10), (9, 10), (10, 10), (1978, 1978), (12, 7)):
-            assert np.float32(a.schedule_function(batch_id, num_batch)) == \
-                np.float32(b.schedule_function(batch_id, num_batch)), (kind, batch_id, num_batch)
+    assert observe_lr_schedules(gv.optimizer) == ref["lr_schedules"]
     with pytest.raises(ValueError):  # the reference CHECK-fails (aborts the process) on the same input
         gv.optimizer.LRSchedule("cosine")
 
@@ -150,69 +175,87 @@ def write_graph(path, rng, num_vertex, num_edge, weighted, comment):
             out.write(line + "\n")
 
 
-@pytest.mark.parametrize("as_undirected", [True, False])
-@pytest.mark.parametrize("normalization", [False, True])
-@pytest.mark.parametrize("weighted", [False, True])
-def test_graph_loader_matches_the_reference_object(ref, gv, tmp_path, as_undirected, normalization, weighted):
+def observe_graph(graph, tmp_path, save_modes=((True, False),), sample=None):
+    """counts, flags, the id map and digests of what save(weighted, anonymous) writes in each mode"""
+    out = {"counts": [graph.num_vertex, graph.num_edge], "flags": [graph.as_undirected, graph.normalization],
+           "id2name": names_digest(list(graph.id2name)), "saved": []}
+    if sample:
+        out["name2id"] = [graph.name2id[name] for name in list(graph.id2name)[::sample]]
+    for mode, (weighted, anonymous) in enumerate(save_modes):
+        path = str(tmp_path / ("saved%d.txt" % mode))
+        graph.save(path, weighted, anonymous)
+        out["saved"].append(file_digest(path))
+    return out
+
+
+LOADER_MODES = ((True, False), (False, False), (True, True), (False, True))
+LOADER_CASES = [(u, n, w) for w in (False, True) for n in (False, True) for u in (True, False)]
+
+
+def observe_graph_loader(graph_class, tmp_path, as_undirected, normalization, weighted):
     """Same edge list through both loaders: ids in order of first appearance, edge counts, and a
     byte-identical save() in every mode (instance/graph.cuh:137-277)."""
     rng = np.random.default_rng(7 + 2 * as_undirected + normalization)
     source = str(tmp_path / "edges.txt")
     write_graph(source, rng, 300, 2500, weighted, comment=True)
-    theirs, ours = ref.graph.Graph_j(), gv.graph.Graph()
-    theirs.load(source, as_undirected, normalization)
-    ours.load(source, as_undirected, normalization)
-    assert (theirs.num_vertex, theirs.num_edge) == (ours.num_vertex, ours.num_edge)
-    assert (theirs.as_undirected, theirs.normalization) == (ours.as_undirected, ours.normalization)
-    assert list(theirs.id2name) == list(ours.id2name)
-    for name in list(theirs.id2name)[::37]:
-        assert theirs.name2id[name] == ours.name2id[name]
-    for mode, (w, anonymous) in enumerate(((True, False), (False, False), (True, True), (False, True))):
-        a, b = str(tmp_path / ("ref%d.txt" % mode)), str(tmp_path / ("ours%d.txt" % mode))
-        theirs.save(a, w, anonymous)
-        ours.save(b, w, anonymous)
-        assert filecmp.cmp(a, b, shallow=False), (w, anonymous)
+    graph = graph_class()
+    graph.load(source, as_undirected, normalization)
+    return observe_graph(graph, tmp_path, LOADER_MODES, sample=37)
 
 
-def test_edge_list_overloads_match_the_reference_object(ref, gv, tmp_path):
+def loader_key(as_undirected, normalization, weighted):
+    return "u%d_n%d_w%d" % (as_undirected, normalization, weighted)
+
+
+@pytest.mark.parametrize("as_undirected", [True, False])
+@pytest.mark.parametrize("normalization", [False, True])
+@pytest.mark.parametrize("weighted", [False, True])
+def test_graph_loader_matches_the_reference_object(ref, gv, tmp_path, as_undirected, normalization, weighted):
+    ours = observe_graph_loader(gv.graph.Graph, tmp_path, as_undirected, normalization, weighted)
+    assert ours == ref["graph_loader"][loader_key(as_undirected, normalization, weighted)]
+
+
+def observe_edge_list_overloads(graph_class, tmp_path):
     rng = np.random.default_rng(11)
     pairs = [("v%d" % u, "v%d" % v) for u, v in rng.integers(0, 50, (400, 2))]
     triples = [(u, v, float(0.5 + 0.5 * (i % 5))) for i, (u, v) in enumerate(pairs)]
+    out = []
     for edges in (pairs, triples):
         for as_undirected in (True, False):
-            theirs, ours = ref.graph.Graph_j(), gv.graph.Graph()
-            theirs.load(edges, as_undirected, False)
-            ours.load(edges, as_undirected, False)
-            assert (theirs.num_vertex, theirs.num_edge) == (ours.num_vertex, ours.num_edge)
-            assert list(theirs.id2name) == list(ours.id2name)
-            a, b = str(tmp_path / "a.txt"), str(tmp_path / "b.txt")
-            theirs.save(a, True, False)
-            ours.save(b, True, False)
-            assert filecmp.cmp(a, b, shallow=False)
+            graph = graph_class()
+            graph.load(edges, as_undirected, False)
+            out.append(observe_graph(graph, tmp_path))
+    return out
 
 
-def test_custom_delimiters_and_comment_prefix(ref, gv, tmp_path):
+def test_edge_list_overloads_match_the_reference_object(ref, gv, tmp_path):
+    assert observe_edge_list_overloads(gv.graph.Graph, tmp_path) == ref["edge_list_overloads"]
+
+
+def observe_custom_delimiters(graph_class, tmp_path):
     source = str(tmp_path / "csv.txt")
     with open(source, "w") as out:
         out.write("% matrix market style comment\n")
         out.write("a,b,2\nb,c,1.5 % note\nc,a,0.5\na,d,1\n")
-    theirs, ours = ref.graph.Graph_j(), gv.graph.Graph()
-    theirs.load(source, True, False, ",\r\n", "%")
-    ours.load(source, True, False, ",\r\n", "%")
-    assert (theirs.num_vertex, theirs.num_edge) == (ours.num_vertex, ours.num_edge) == (4, 4)
-    assert list(theirs.id2name) == list(ours.id2name)
-    a, b = str(tmp_path / "a.txt"), str(tmp_path / "b.txt")
-    theirs.save(a, True, False)
-    ours.save(b, True, False)
-    assert filecmp.cmp(a, b, shallow=False)
+    graph = graph_class()
+    graph.load(source, True, False, ",\r\n", "%")
+    return observe_graph(graph, tmp_path)
+
+
+def test_custom_delimiters_and_comment_prefix(ref, gv, tmp_path):
+    ours = observe_custom_delimiters(gv.graph.Graph, tmp_path)
+    assert ours["counts"] == [4, 4]
+    assert ours == ref["custom_delimiters"]
+
+
+def observe_toy_graph(graph_class):
+    graph = graph_class()
+    graph.load(TOY, True, False)
+    return {"counts": [graph.num_vertex, graph.num_edge], "id2name": list(graph.id2name)}
 
 
 def test_toy_graph_golden_is_what_the_reference_loads(ref, gv):
-    theirs, ours = ref.graph.Graph_j(), gv.graph.Graph()
-    theirs.load(TOY, True, False)
-    ours.load(TOY, True, False)
-    assert (theirs.num_vertex, theirs.num_edge) == (ours.num_vertex, ours.num_edge)
-    assert list(theirs.id2name) == list(ours.id2name)
+    assert observe_toy_graph(gv.graph.Graph) == ref["toy_graph"]
 
 
 # ---- KnowledgeGraph (instance/knowledge_graph.cuh:67-284) ------------------------------------------
@@ -239,46 +282,45 @@ def kg_flatten(gv, graph):
 
 
 def test_knowledge_graph_surface(ref, gv):
-    assert public(ref.graph.KnowledgeGraph_j) <= public(gv.graph.KnowledgeGraph)
-    theirs = doc_signature(ref.graph.KnowledgeGraph_j.save)
+    assert set(ref["public"]["KnowledgeGraph_j"]) <= public(gv.graph.KnowledgeGraph)
+    theirs = doc_signature(ref["docs"]["KnowledgeGraph_j.save"])
     ours = our_signature(gv.graph.KnowledgeGraph.save)
     assert [n for n, _ in theirs] == [n for n, _ in ours]
     for (name, a), (_, b) in zip(theirs, ours):
         assert same_default(a, b, gv), (name, a, b)
 
 
-@pytest.mark.parametrize("normalization", [False, True])
-@pytest.mark.parametrize("weighted", [False, True])
-def test_knowledge_graph_loader_matches_the_reference_object(ref, gv, tmp_path, normalization, weighted):
+def load_kg_loader_case(kg_class, tmp_path, normalization, weighted):
     rng = np.random.default_rng(3 + normalization)
     source = str(tmp_path / "triplets.txt")
     write_triplets(source, rng, 120, 9, 1500, weighted)
-    theirs, ours = ref.graph.KnowledgeGraph_j(), gv.graph.KnowledgeGraph()
-    theirs.load(source, normalization)
-    ours.load(source, normalization)
-    assert (theirs.num_vertex, theirs.num_edge, theirs.num_relation) == (ours.num_vertex, ours.num_edge,
-                                                                         ours.num_relation)
-    assert theirs.normalization == ours.normalization
-    assert list(theirs.id2entity) == list(ours.id2entity)
-    assert list(theirs.id2relation) == list(ours.id2relation)
-    for name in list(theirs.id2entity)[::17]:
-        assert theirs.entity2id[name] == ours.entity2id[name]
-    for name in theirs.id2relation:
-        assert theirs.relation2id[name] == ours.relation2id[name]
+    graph = kg_class()
+    graph.load(source, normalization)
+    return graph
+
+
+def observe_kg(graph):
+    return {"counts": [graph.num_vertex, graph.num_edge, graph.num_relation], "normalization": graph.normalization,
+            "id2entity": names_digest(list(graph.id2entity)), "id2relation": list(graph.id2relation),
+            "entity2id": [graph.entity2id[name] for name in list(graph.id2entity)[::17]],
+            "relation2id": [graph.relation2id[name] for name in graph.id2relation],
+            "repr_tail": repr(graph).splitlines()[-2:]}
+
+
+@pytest.mark.parametrize("normalization", [False, True])
+@pytest.mark.parametrize("weighted", [False, True])
+def test_knowledge_graph_loader_matches_the_reference_object(ref, gv, tmp_path, normalization, weighted):
+    theirs = ref["kg_loader"]["n%d_w%d" % (normalization, weighted)]
+    ours = load_kg_loader_case(gv.graph.KnowledgeGraph, tmp_path, normalization, weighted)
+    assert observe_kg(ours) == theirs["graph"]
     # anonymous save of the reference = head, tail, int(weight) in flatten order: pins heads, tails and order;
     # (its third column is the weight by mistake, knowledge_graph.cuh:275)
-    path = str(tmp_path / "ref.txt")
-    theirs.save(path, True)
-    columns = np.loadtxt(path, dtype=np.int64, ndmin=2)
     h, t, r, w, _ = kg_flatten(gv, ours)
-    np.testing.assert_array_equal(columns[:, 0], h)
-    np.testing.assert_array_equal(columns[:, 1], t)
-    np.testing.assert_array_equal(columns[:, 2], w.astype(np.int64))  # float -> unsigned long long truncation
+    assert [int_digest(h), int_digest(t), int_digest(w.astype(np.int64))] == theirs["anonymous_columns"]
     assert "#entity: %d, #relation: %d" % (ours.num_vertex, ours.num_relation) in repr(ours)
-    assert repr(theirs).splitlines()[-2:] == repr(ours).splitlines()[-2:]
 
 
-def test_knowledge_graph_save_is_byte_identical_where_the_reference_is_well_defined(ref, gv, tmp_path):
+def observe_kg_save(kg_class, tmp_path):
     """weights equal to the relation ids make the reference's `relation = weight` slip invisible"""
     rng = np.random.default_rng(9)
     relations = ["r%d" % i for i in range(6)]
@@ -288,15 +330,20 @@ def test_knowledge_graph_save_is_byte_identical_where_the_reference_is_well_defi
     for _ in range(300):
         r = int(rng.integers(0, 6))
         triplets.append(("e%d" % rng.integers(0, 40), relations[r], "e%d" % rng.integers(0, 40), float(r)))
-    theirs, ours = ref.graph.KnowledgeGraph_j(), gv.graph.KnowledgeGraph()
-    theirs.load(triplets, False)
-    ours.load(triplets, False)
-    assert list(theirs.id2relation) == list(ours.id2relation) == relations
+    graph = kg_class()
+    graph.load(triplets, False)
+    out = {"id2relation": list(graph.id2relation), "saved": []}
     for anonymous in (False, True):
-        a, b = str(tmp_path / "a.txt"), str(tmp_path / "b.txt")
-        theirs.save(a, anonymous)
-        ours.save(b, anonymous)
-        assert filecmp.cmp(a, b, shallow=False), anonymous
+        path = str(tmp_path / "saved.txt")
+        graph.save(path, anonymous)
+        out["saved"].append(file_digest(path))
+    return out
+
+
+def test_knowledge_graph_save_is_byte_identical_where_the_reference_is_well_defined(ref, gv, tmp_path):
+    ours = observe_kg_save(gv.graph.KnowledgeGraph, tmp_path)
+    assert ours["id2relation"] == ["r%d" % i for i in range(6)]
+    assert ours == ref["kg_save"]
 
 
 def test_knowledge_graph_normalization_weights(ref, gv, tmp_path):
@@ -352,24 +399,28 @@ def write_corpus(path, rng, vocabulary, lines):
             out.write(text + "\n")
 
 
-@pytest.mark.parametrize("window,min_count,normalization", [(5, 5, False), (2, 1, False), (7, 3, True)])
-def test_word_graph_loader_matches_the_reference_object(ref, gv, tmp_path, window, min_count, normalization):
+WORD_CASES = [(5, 5, False), (2, 1, False), (7, 3, True)]
+
+
+def observe_word_graph(word_class, tmp_path, window, min_count, normalization):
     """Vocabulary (ids by first appearance, min_count filter), co-occurrence counts and -- because the out-edges of
     a vertex are emitted in the iteration order of an unordered_map -- the edge ORDER: save() must be byte-identical."""
     rng = np.random.default_rng(11 + window)
     corpus = str(tmp_path / "corpus.txt")
     write_corpus(corpus, rng, 150, 400)
-    theirs, ours = ref.graph.WordGraph_j(), gv.graph.WordGraph()
-    theirs.load(corpus, window, min_count, normalization)
-    ours.load(corpus, window, min_count, normalization)
-    assert [n for n, _ in doc_signature(theirs.load)] == [n for n, _ in our_signature(gv.graph.WordGraph.load)]
-    assert (theirs.num_vertex, theirs.num_edge) == (ours.num_vertex, ours.num_edge)
-    assert ours.num_vertex > 20 and ours.num_edge > 100
-    assert (theirs.as_undirected, theirs.normalization) == (ours.as_undirected, ours.normalization) == (True, normalization)
-    assert list(theirs.id2name) == list(ours.id2name)
-    for mode, (weighted, anonymous) in enumerate(((True, False), (False, True))):
-        a, b = str(tmp_path / ("ref%d.txt" % mode)), str(tmp_path / ("ours%d.txt" % mode))
-        theirs.save(a, weighted, anonymous)
-        ours.save(b, weighted, anonymous)
-        assert filecmp.cmp(a, b, shallow=False), (weighted, anonymous)
-    assert repr(ours).splitlines()[0] == repr(theirs).splitlines()[0] == "WordGraph<uint32>"
+    graph = word_class()
+    graph.load(corpus, window, min_count, normalization)
+    return dict(observe_graph(graph, tmp_path, ((True, False), (False, True))),
+                repr_head=repr(graph).splitlines()[0])
+
+
+@pytest.mark.parametrize("window,min_count,normalization", WORD_CASES)
+def test_word_graph_loader_matches_the_reference_object(ref, gv, tmp_path, window, min_count, normalization):
+    theirs = ref["word_graph"]["%d_%d_%d" % (window, min_count, normalization)]
+    assert [n for n, _ in doc_signature(ref["docs"]["WordGraph_j.load"])] == \
+        [n for n, _ in our_signature(gv.graph.WordGraph.load)]
+    ours = observe_word_graph(gv.graph.WordGraph, tmp_path, window, min_count, normalization)
+    assert ours["counts"][0] > 20 and ours["counts"][1] > 100
+    assert ours["flags"] == [True, normalization]
+    assert ours["repr_head"] == "WordGraph<uint32>"
+    assert ours == theirs
